@@ -2,6 +2,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one process per GPU)
   python bench.py --impl reference --steps K --warmup W    # CPU restatement of the reference path (oracle)
+  python bench.py --steps K --warmup W --dump-outputs bench_outputs   # + the last timed step's outputs as .npy
 
 Headline workload (config.workload) = BASELINE.json configs[1]: ddpm-mel-32seq-512.cfg (TransformerDDPM L6/H8/K2/M2048,
 C=42 after slice-mel-512), batch 128 per GPU, one optimizer step = device threefry draws + q_sample + forward +
@@ -18,6 +19,16 @@ the same global batch on one GPU).
 
 The reference arm and the cpu_baseline leg run the CPU oracle (oracle/, torch fp32) and never import the product
 package, so no product shared library is mapped into a reference process.
+
+--dump-outputs DIR writes what the last of the K timed steps handed back to its caller as DIR/<name>.npy (rank 0):
+  train   loss.npy, grad_norm.npy (the step's global mean loss and clipped gradient norm) and params.npy (the updated
+          parameters, flattened in layout order)
+  sample  samples.npy (the (N, 32, C) state after the reverse step)
+Inputs are seeded, so two builds run with the same arguments can be compared array for array.  An array of more than
+DUMP_MAX_VALUES values is stored as its values at DUMP_MAX_VALUES fixed, seeded positions (params.npy of the base model
+is such a sample), which keeps a dump well under 64 MB.  The backward pass accumulates some gradients with float
+atomics, so train dumps agree to a tolerance, not bit for bit: two runs of one build with --steps 20 --warmup 5 (B200,
+1000 W power limit) differed by 8e-5 relative in loss and 1.6e-4 in the rel-L2 of params.
 """
 from __future__ import annotations
 
@@ -47,6 +58,27 @@ MODELS = {
     "base_c512": dict(channels=512, **BASE),     # --slice_ckpt='' variant
 }
 HEADLINE_WL = "train ddpm-mel-32seq-512.cfg (TransformerDDPM L6 H8 K2 M2048 C42), batch 128/GPU"
+DUMP_MAX_VALUES = 1 << 22       # per dumped array: 16 MiB of float32
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes each array as out_dir/<name>.npy in float32 (float64 stays float64).  An array with more than
+    DUMP_MAX_VALUES values is replaced by its flattened values at DUMP_MAX_VALUES positions drawn without replacement by
+    np.random.default_rng(0) and sorted, so the same positions are kept in every run."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)
+        a = a if a.dtype == np.float64 else a.astype(np.float32)
+        if a.size > DUMP_MAX_VALUES:
+            pos = np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_VALUES, replace=False))
+            a = a.reshape(-1)[pos]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    print(f"bench: wrote {', '.join(f'{n}.npy' for n in arrays)} to {out_dir}", file=sys.stderr, flush=True)
+
+
+def flat_params(named: dict) -> np.ndarray:
+    """Parameter tensors (name -> array, in layout order) as one flat float32 vector."""
+    return np.concatenate([np.asarray(v, np.float32).reshape(-1) for v in named.values()])
 
 
 def synthetic_batch(batch: int, seed: int, channels: int = 42):
@@ -154,9 +186,9 @@ class CpuTrainStep:
 
     def step(self) -> float:
         t0 = time.perf_counter()
-        (self.p, self.mom, self.var), _, _, _ = self.O.train_step(self.m["arch"], self.p, self.mom, self.var, self.n,
-                                                                  self.x0, self.used, self.eps, 1e-3,
-                                                                  model_kw=_oracle_kw(self.m))
+        (self.p, self.mom, self.var), self.loss, self.grad_norm, _ = self.O.train_step(
+            self.m["arch"], self.p, self.mom, self.var, self.n, self.x0, self.used, self.eps, 1e-3,
+            model_kw=_oracle_kw(self.m))
         self.n += 1
         return time.perf_counter() - t0
 
@@ -198,6 +230,10 @@ def run_reference(args):
     for _ in range(args.warmup):
         job.step()
     times = [job.step() for _ in range(args.steps)]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"loss": np.atleast_1d(np.asarray(job.loss, np.float32)),
+                                         "grad_norm": np.atleast_1d(np.asarray(job.grad_norm, np.float32)),
+                                         "params": flat_params({k: v.detach().numpy() for k, v in job.p.items()})})
     sb = job.batch
     ms = 1e3 * float(np.mean(times))
     value = sb / (ms / 1e3)
@@ -320,8 +356,12 @@ def make_train(ctx: Ctx, model: str, B: int):
         ev.record()
         loss_done[j] = ev
 
+    def outputs():
+        # what train_step hands its caller (global mean loss, clipped gradient norm) and the parameters it updated
+        return {"loss": eng.loss_mean, "grad_norm": eng.grad_norm, "params": flat_params(eng.flat_to_dict(eng.params))}
+
     return dict(eng=eng, cfg=cfg, units=B, flops=3.0 * cfg.flops_fwd_per_sample() * B, resident=step_resident,
-                e2e=step_e2e, h2d=x_host.numel() * 4, d2h=4, tokens=B * 32, x_host=x_host)
+                e2e=step_e2e, h2d=x_host.numel() * 4, d2h=4, tokens=B * 32, x_host=x_host, outputs=outputs)
 
 
 def make_sample(ctx: Ctx, model: str, N: int):
@@ -347,7 +387,7 @@ def make_sample(ctx: Ctx, model: str, N: int):
         torch.cuda.current_stream().synchronize()
 
     return dict(eng=eng, cfg=cfg, units=N, flops=cfg.flops_fwd_per_sample() * N, resident=step_resident, e2e=step_e2e,
-                h2d=x_host.numel() * 4, d2h=x_host.numel() * 4, tokens=N * 32)
+                h2d=x_host.numel() * 4, d2h=x_host.numel() * 4, tokens=N * 32, outputs=lambda: {"samples": x_dev})
 
 
 def extra_entry(ctx: Ctx, name: str, what: str, job, steps: int, warmup: int):
@@ -423,6 +463,8 @@ def run_gpu(args):
     ms_step, launches = ctx.timed(job["resident"], args.steps, args.warmup, eng)
     clocks.stop_flag.set()
     clocks.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, job["outputs"]())     # before the e2e leg runs further steps
     ms_e2e, _ = ctx.timed(job["e2e"], args.steps, max(3, args.warmup // 2), eng)
 
     units, flops_step = job["units"], job["flops"]
@@ -515,7 +557,11 @@ def main():
     ap.add_argument("--cta-group", dest="cta_group", type=int, default=2)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra BASELINE configs")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
